@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native SpMV + Krylov hot path.
 
-  python bench.py --gpus N --steps K --warmup W [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 A "step" is one CSR SpMV  y = A x  of BASELINE.json configs[1]: random CSR fp64,
 n = 10 000 000, nnz = 150 000 000 (15 distinct uniform columns per row), synthetic data from
@@ -94,6 +94,39 @@ class ClockSampler:
                 "samples": len(self.samples)}
 
 
+class OutputDump:
+    """--dump-outputs DIR: what every timed leg computed in its last step, as DIR/<name>.npy.  Each
+    leg keeps a sample of its result vector at positions drawn by a seeded generator (the same in
+    every run, 64 MB in all), so two builds run with the same arguments compare output for output."""
+    MAX_BYTES = 64 << 20
+
+    def __init__(self, path, world, stream):
+        self.path, self.world, self.stream, self.arrays = path, world, stream, {}
+
+    def take(self, name, local, r0, n_total, k):
+        """local = rows [r0, r0 + local.numel()) of an n_total-row result; every rank calls this"""
+        import torch
+        import torch.distributed as dist
+        k = min(k, n_total)
+        idx = np.sort(np.random.default_rng(1).choice(n_total, k, replace=False))
+        with torch.cuda.stream(self.stream):
+            idx = torch.from_numpy(idx).to(local.device)
+            mine = (idx >= r0) & (idx < r0 + local.numel())
+            out = torch.zeros(k, dtype=local.dtype, device=local.device)
+            out[mine] = local.reshape(-1)[idx[mine] - r0]
+            if self.world > 1:  # each position is owned by one rank, the others add zeros
+                dist.all_reduce(out)
+            self.arrays[name] = out.cpu().numpy()
+
+    def write(self):
+        total = sum(a.nbytes for a in self.arrays.values())
+        if total > self.MAX_BYTES:
+            raise RuntimeError("--dump-outputs: %d bytes exceed %d" % (total, self.MAX_BYTES))
+        os.makedirs(self.path, exist_ok=True)
+        for name, a in self.arrays.items():
+            np.save(os.path.join(self.path, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------ CPU arm (reference OMP)
 def cfg2_on_host():
     """the FULL cfg2 matrix + x as numpy arrays (generated on the GPU when there is one: the
@@ -114,10 +147,10 @@ def cfg2_on_host():
     return rp, ci, va, W.vector(N_ROWS)
 
 
-def cpu_reference_spmv(mat, min_reps, min_seconds=2.0):
+def cpu_reference_spmv(mat, min_reps, min_seconds=2.0, reps=None):
     """the reference's OMP executor (oracle/_ref) on the full cfg2 -- same config as the GPU arm --
     or, if that was not built, the oracle port.  Reference methodology (benchmark/utils/timer):
-    warm-up, then >= min_reps repetitions and >= min_seconds."""
+    warm-up, then >= min_reps repetitions and >= min_seconds; exactly `reps` repetitions when given."""
     rp, ci, va, x = mat
     nnz = len(va)
     n = len(rp) - 1
@@ -125,13 +158,15 @@ def cpu_reference_spmv(mat, min_reps, min_seconds=2.0):
     if ref.available():
         cores = ref.use_physical_cores()
         _, sec1 = ref.spmv("csr", rp, ci, va, x, N_ROWS, exec_kind=1, reps=2)  # warm-up, first touch
-        reps = int(max(min_reps, min(200, min_seconds / max(sec1, 1e-6))))
+        if reps is None:
+            reps = int(max(min_reps, min(200, min_seconds / max(sec1, 1e-6))))
         _, sec = ref.spmv("csr", rp, ci, va, x, N_ROWS, exec_kind=1, reps=reps)
         kind = "reference"
     else:
         from oracle import oracle
         y = np.zeros(n)
-        reps = max(1, min_reps // 4)
+        if reps is None:
+            reps = max(1, min_reps // 4)
         t0 = time.perf_counter()
         for _ in range(reps):
             oracle.call("orc_csr_spmv_f64_i32", n, N_ROWS, nnz, rp, ci, va, x, 1, 1, y, 1)
@@ -149,7 +184,7 @@ def cpu_reference_spmv(mat, min_reps, min_seconds=2.0):
 def run_reference_arm(args, rank):
     if rank != 0:
         return
-    b = cpu_reference_spmv(cfg2_on_host(), max(1, min(args.steps, 200)))
+    b = cpu_reference_spmv(cfg2_on_host(), args.steps, reps=args.steps)
     line = {
         "impl": "reference", "metric": "csr_spmv_fp64_gflops", "value": b["value"],
         "unit": "GFLOP/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -180,6 +215,7 @@ def run_gpu_arm(args, rank, world):
     ex = api.HostExecutor(local)  # C++ host layer (gko_b200.hpp) over the C ABI
     dev = ex.device
     hl = api._host()
+    dump = OutputDump(args.dump_outputs, world, ex.stream) if args.dump_outputs else None
 
     def timed(fn, n):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -265,6 +301,8 @@ def run_gpu_arm(args, rank, world):
         l0 = ex.launch_count()
         ms_total = timed(step, args.steps)
         launches = ex.launch_count() - l0
+        if dump:
+            dump.take("csr_spmv_cfg2_y", y_t, r0, N_ROWS, 2 << 20)
         for _ in range(3):
             kernel_step()
         ms_kernel = timed(kernel_step, args.steps) / args.steps  # dominant kernel alone
@@ -297,6 +335,8 @@ def run_gpu_arm(args, rank, world):
                                                        "to 1e-13 relative (checked in this run)"}
                 if ms_ov < ms_total:
                     ms_total, launches = ms_ov, launches_ov
+                    if dump:
+                        dump.take("csr_spmv_cfg2_y", y_t, r0, N_ROWS, 2 << 20)
                     halo_path += "; exchange and SpMV pipelined by owner block (opt-in mode, 1e-13-equal row sums)"
                 else:
                     A.set_overlap(False)
@@ -396,6 +436,8 @@ def run_gpu_arm(args, rank, world):
         for _ in range(3):
             bstep()
         ms_b = timed(bstep, args.steps) / args.steps
+        if dump:
+            dump.take("csr_spmv_cfg2_banded_y", yb, 0, N_ROWS, 1 << 20)
         bbytes = W.spmv_bytes(N_ROWS, N_ROWS, bva.numel())
         twin = {"workload": "banded twin of cfg2: n=%d, columns row-7..row+7, nnz=%d" % (N_ROWS, bva.numel()),
                 "ms_per_step": ms_b, "gflops": 2.0 * bva.numel() / (ms_b * 1e-3) / 1e9,
@@ -419,6 +461,8 @@ def run_gpu_arm(args, rank, world):
         for _ in range(3):
             zstep()
         ms_z = timed(zstep, args.steps) / args.steps
+        if dump:
+            dump.take("csr_spmv_cfg2_zipf_y", yz, 0, N_ROWS, 1 << 20)
         zbytes = W.spmv_bytes(N_ROWS, N_ROWS, zva.numel())
         with torch.cuda.stream(ex.stream):
             zl = (zrp[1:] - zrp[:-1])
@@ -436,10 +480,12 @@ def run_gpu_arm(args, rank, world):
     del x_full
 
     # ------------------------------------------------------------------------------ CG
-    cg = run_cg(args, rank, world, ex, dev, timed_events=True)
+    cg = run_cg(args, rank, world, ex, dev, timed_events=True, dump=dump)
 
     if rank != 0:
         return
+    if dump:
+        dump.write()
     cpu = cpu_reference_spmv(host_mat, 10) if host_mat is not None else None
     line = {
         "metric": "csr_spmv_fp64_gflops", "value": value, "unit": "GFLOP/s", "n_gpus": world,
@@ -466,7 +512,7 @@ def run_gpu_arm(args, rank, world):
     print(json.dumps(line))
 
 
-def run_cg(args, rank, world, ex, dev, timed_events=True):
+def run_cg(args, rank, world, ex, dev, timed_events=True, dump=None):
     """CG iterations/s: N == 1 -> BASELINE configs[2] (7-pt Laplacian 200^3 + scalar Jacobi, to
     1e-8) AND configs[4] (400^3, 200 iterations); N > 1 -> configs[4] row-sharded (z-slabs)."""
     import torch
@@ -504,6 +550,8 @@ def run_cg(args, rank, world, ex, dev, timed_events=True):
         s.apply(bd, xd)  # warm-up solve (builds the plan + graph)
         x.zero_()
         ms = wall(lambda: s.apply(bd, xd))
+        if dump:
+            dump.take("cg_cfg3_x", x, 0, n, 1 << 20)
         # true relative residual
         r = b.clone()
         rd = api.host_dense(ex, r)
@@ -547,6 +595,8 @@ def run_cg(args, rank, world, ex, dev, timed_events=True):
         setup_s = time.perf_counter() - t0
         x.zero_()
         ms = wall(lambda: s.apply(bd, xd))
+        if dump:
+            dump.take("gmres_cfg4_x", x, 0, n, 1 << 20)
         r = b.clone()
         rd = api.host_dense(ex, r)
         one = api.host_dense(ex, torch.ones(1, dtype=torch.float32, device=dev))
@@ -618,6 +668,8 @@ def run_cg(args, rank, world, ex, dev, timed_events=True):
         res = {}
         ms = wall(lambda: res.update(it=A.cg_apply(b, x)[0]))
         done, ghosts = res["it"], A.n_ghost
+    if dump:
+        dump.take("cg_cfg5_x", x, r0, n, 1 << 20)
     # TRUE residual ||b - A x|| / ||b|| of the timed solve, identical code path for every N
     # (a wrong halo inside the CG graph would show here); compared with the reference's
     # 200-iteration value (tests/golden/fullsize_reference.json) at the full size
@@ -682,7 +734,13 @@ def main():
     ap.add_argument("--no-gmres", action="store_true", help="skip the GMRES + block-Jacobi leg")
     ap.add_argument("--no-twin", action="store_true", help="skip the banded twin of cfg2")
     ap.add_argument("--small-cg", action="store_true", help="160^3 instead of 400^3 for the cfg5 leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of every timed leg's result to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the GPU legs; --impl reference has none")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     if args.impl == "reference":

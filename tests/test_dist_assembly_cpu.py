@@ -14,6 +14,7 @@ import pytest
 
 from tests import dist_driver as D
 from tests import helpers as H
+from tests import reference
 from tests.test_kernel_sources_cpu import KernelSourceBackend
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -50,7 +51,10 @@ TYPES = [("i32", "i32"), ("i32", "i64"), ("i64", "i64")]
 
 
 def eq(a, b):
-    np.testing.assert_array_equal(np.asarray(a), np.asarray(b))
+    if isinstance(b, reference.Digest):  # a recorded answer of the reference
+        assert reference.equal(a, b, equal_nan=True)
+    else:
+        np.testing.assert_array_equal(np.asarray(a), np.asarray(b))
 
 
 # --------------------------------------------------------------------------------- partition
@@ -209,20 +213,9 @@ def random_mapping(rng, n, num_parts, run):
     return np.array(out[:n], np.int32)
 
 
-def ref_or_skip():
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not built")
-    try:
-        ref.lib().refshim_partition
-    except AttributeError:
-        pytest.skip("oracle/_ref predates the distributed shim functions")
-    return ref
-
-
 @pytest.mark.parametrize("seed", range(6))
 def test_partition_matches_reference(be, seed):
-    ref = ref_or_skip()
+    ref = reference
     rng = np.random.default_rng(seed)
     num_parts = int(rng.integers(1, 9))
     mapping = random_mapping(rng, int(rng.integers(1, 400)), num_parts, 7)
@@ -250,7 +243,7 @@ def test_partition_matches_reference(be, seed):
 
 @pytest.mark.parametrize("seed", range(6))
 def test_separate_and_index_map_match_reference(be, seed):
-    ref = ref_or_skip()
+    ref = reference
     rng = np.random.default_rng(100 + seed)
     num_parts = int(rng.integers(2, 7))
     nrows, ncols = int(rng.integers(20, 200)), int(rng.integers(20, 200))
@@ -270,15 +263,16 @@ def test_separate_and_index_map_match_reference(be, seed):
             eq(got, want)
         for got, want in zip(s["non_local"], nonloc):
             eq(got, want)
+        nonloc_cols = np.asarray(s["non_local"][1], np.int64)  # = the reference's, checked above
         # kept = all entries of the owned rows in input order
         owned = row_map[rows] == part
         eq(s["kept"][1], cols[owned])
         eq(s["kept"][2], vals[owned])
         # the index map of the non-local columns
-        im = D.IndexMap(be, cp, part, nonloc[1])
+        im = D.IndexMap(be, cp, part, nonloc_cols)
         q = rng.integers(0, ncols, 50)
         for space in (0, 1, 2):
-            r = ref.index_map(col_map, num_parts, part, nonloc[1], space, q)
+            r = ref.index_map(col_map, num_parts, part, nonloc_cols, space, q)
             eq(im.remote_global, r["remote_global"])
             eq(im.remote_local, r["remote_local"])
             ids, sizes = im.target_ids()
@@ -350,9 +344,7 @@ def test_vector_build_local_matches_reference(be, lt, gt, seed):
                 want[local_of[r], c] = v
         eq(got, want)
         if (lt, gt) == ("i32", "i64"):
-            ref = ref_or_skip()
-            if hasattr(ref.lib(), "refshim_vector_build_local"):
-                eq(got, ref.vector_build_local((nrows, ncols), rows, cols, vals, mapping, num_parts, p))
+            eq(got, reference.vector_build_local((nrows, ncols), rows, cols, vals, mapping, num_parts, p))
 
 
 def test_kernel_sources_are_race_free_under_real_threads(tmp_path):

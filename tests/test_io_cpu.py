@@ -1,16 +1,14 @@
 """MatrixMarket / Ginkgo-binary I/O of the host layer (ginkgo_b200/host/gko_b200_io.hpp, pure
 C++ without CUDA) against the REAL reference's gko::read_generic_raw / write_raw /
-write_binary_raw (core/base/mtx_io.cpp) through oracle/_ref.  CPU only: the header is
-compiled into tests/cpp/io_check with plain g++."""
+write_binary_raw (core/base/mtx_io.cpp) through oracle/_ref, or its recorded answers
+(tests/reference.py).  CPU only: the header is compiled into tests/cpp/io_check with plain g++."""
 import os
 import subprocess
 
 import numpy as np
 import pytest
 
-ref = pytest.importorskip("oracle.ref")
-if not ref.available():
-    pytest.skip("oracle/_ref not built (needs /root/reference at build time)", allow_module_level=True)
+from tests import reference as ref
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 

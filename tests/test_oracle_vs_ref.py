@@ -1,18 +1,15 @@
 """Pins the oracle (oracle/liboracle.so, our C restatement) against the REAL reference:
 oracle/_ref is the reference's own core + ReferenceExecutor + OmpExecutor sources compiled
 in place (oracle/ref_build/Makefile) and driven through its public API (oracle/ref_shim.cpp).
-Runs wherever oracle/_ref exists (this container, and the GPU box via the shipped .so)."""
+Where oracle/_ref is not built, the reference's recorded answers stand in (tests/reference.py)."""
 import ctypes
 
 import numpy as np
 import pytest
 
 from tests import helpers as H
+from tests import reference as ref
 from tests.helpers import VT
-
-ref = pytest.importorskip("oracle.ref")
-if not ref.available():
-    pytest.skip("oracle/_ref not built (needs /root/reference at build time)", allow_module_level=True)
 from oracle import oracle  # noqa: E402
 
 import workloads as W  # noqa: E402
@@ -29,16 +26,16 @@ def test_spmv_bit_identical_to_reference(orc, vt, fmt):
         y_ref, _ = ref.spmv(fmt, rp, ci, va, x, m)
         y = np.zeros((n, nrhs), VT[vt])
         orc("csr_spmv_%s_i32" % vt, n, m, len(va), rp, ci, va, x, nrhs, nrhs, y, nrhs)
-        assert np.array_equal(y, y_ref)
+        assert ref.equal(y, y_ref)
         y0 = rng.uniform(-1, 1, (n, nrhs)).astype(VT[vt])
         y_ref, _ = ref.spmv(fmt, rp, ci, va, x, m, alpha=-1.5, beta=0.5, y=y0.copy())
         y = y0.copy()
         orc("csr_advanced_spmv_%s_i32" % vt, n, m, len(va), rp, ci, va, np.array([-1.5], VT[vt]), x,
             nrhs, nrhs, np.array([0.5], VT[vt]), y, nrhs)
         if fmt in ("csr", "ell", "sellp"):
-            assert np.array_equal(y, y_ref)
+            assert ref.equal(y, y_ref)
         else:  # coo/hybrid scale y first, then accumulate: same values up to one rounding
-            assert H.rel_err(y, y_ref) <= H.R[vt]
+            assert ref.close(y, y_ref, H.R[vt])
 
 
 def test_omp_executor_matches_reference_executor():
@@ -46,7 +43,7 @@ def test_omp_executor_matches_reference_executor():
     x = W.vector(len(rp) - 1)
     y0, _ = ref.spmv("csr", rp, ci, va, x, len(rp) - 1, exec_kind=0)
     y1, _ = ref.spmv("csr", rp, ci, va, x, len(rp) - 1, exec_kind=1)
-    assert np.array_equal(y0, y1)
+    assert ref.equal(y0, y1)
 
 
 from tests.helpers import orc_solve  # noqa: E402
@@ -70,7 +67,7 @@ def test_solver_loops_bit_identical_to_reference(kind, precond, vt):
         xo, ito, stop = orc_solve(kind, vt, rp, ci, va, b, x0, precond, jac, max_iters=300,
                                   reduction=red, iter_first=iter_first, krylov_dim=12)
         assert itr == ito
-        assert np.array_equal(xr, xo)
+        assert ref.equal(xo, xr)
         assert stop[0] == (0x80 | 0x40 | (2 if iter_first else 1))
 
 
@@ -85,7 +82,7 @@ def test_gmres_ortho_and_multi_rhs(ortho):
                               krylov_dim=7, ortho=ortho)
     xo, ito, _ = orc_solve("gmres", "f64", rp, ci, va, b, x0, max_iters=60, reduction=1e-6,
                            krylov_dim=7, ortho=ortho)
-    assert itr == ito and np.array_equal(xr, xo)
+    assert itr == ito and ref.equal(xo, xr)
 
 
 @pytest.mark.parametrize("kind", ["cg", "bicgstab"])
@@ -100,7 +97,7 @@ def test_implicit_residual_and_baselines(kind):
                                   baseline=baseline, reduction=1e-7)
         xo, ito, _ = orc_solve(kind, "f64", rp, ci, va, b, x0, max_iters=200, res_kind=res_kind,
                                baseline=baseline, reduction=1e-7)
-        assert itr == ito and np.array_equal(xr, xo), (res_kind, baseline)
+        assert itr == ito and ref.equal(xo, xr), (res_kind, baseline)
 
 
 def test_cfg1_cg_jacobi_matches_survey_probe():
@@ -114,7 +111,7 @@ def test_cfg1_cg_jacobi_matches_survey_probe():
     xr, itr, _, _ = ref.solve("cg", rp, ci, va, b, x0, precond_max_bs=1, max_iters=5000,
                               reduction=1e-8, exec_kind=1)
     assert itr == 579
-    assert H.rel_err(xo, xr) < 1e-12
+    assert ref.close(xo, xr, 1e-12)
 
 
 # ---------------------------------------------------------------- conversions (SURVEY 8f-1)
@@ -141,7 +138,7 @@ def test_convert_to_ell_matches_reference(orc, vt, kind):
     cols = np.full(r["width"] * n, 77, np.int32)
     vals = np.full(r["width"] * n, 7, VT[vt])
     orc("csr_convert_to_ell_%s_i32" % vt, n, rp, ci, va, r["width"], n, cols, vals)
-    assert np.array_equal(cols, r["cols"]) and np.array_equal(vals, r["vals"])
+    assert ref.equal(cols, r["cols"]) and ref.equal(vals, r["vals"])
 
 
 @pytest.mark.parametrize("kind", ["uniform", "skewed", "empty_rows"])
@@ -153,24 +150,16 @@ def test_convert_to_sellp_matches_reference(orc, kind, slice_size, stride_factor
     ns = (n + slice_size - 1) // slice_size
     ss, sl = np.zeros(ns + 1, np.uint64), np.zeros(ns, np.uint64)
     orc("sellp_compute_slice_sets_i32", rp, n, slice_size, stride_factor, ss, sl)
-    assert np.array_equal(ss, r["slice_sets"]) and np.array_equal(sl, r["slice_lengths"])
+    assert ref.equal(ss, r["slice_sets"]) and ref.equal(sl, r["slice_lengths"])
     tot = int(ss[-1]) * slice_size
-    assert tot == len(r["cols"])
-    # slots of rows past num_rows in the last slice are never written by the reference:
-    # compare only what it defines (start from its own buffer for those)
-    cols, vals = r["cols"].copy(), r["vals"].copy()
-    keep_c, keep_v = cols.copy(), vals.copy()
-    cols[:] = 77
-    vals[:] = 7
+    assert (tot,) == r["cols"].shape
+    # slots of rows past num_rows in the last slice are never written (the reference's answers
+    # hold 0 there): compare only what it defines
+    cols, vals = np.full(tot, 77, np.int32), np.full(tot, 7, VT[vt])
     orc("csr_convert_to_sellp_%s_i32" % vt, n, slice_size, ss, sl, rp, ci, va, cols, vals)
-    defined = np.ones(tot, bool)
-    for s in range(ns):
-        for lr in range(slice_size):
-            if s * slice_size + lr >= n:
-                idx = (int(ss[s]) + np.arange(int(sl[s]))) * slice_size + lr
-                defined[idx] = False
-    assert np.array_equal(cols[defined], keep_c[defined])
-    assert np.array_equal(vals[defined], keep_v[defined])
+    defined = ref.sellp_defined(n, slice_size, ss, sl)
+    assert ref.equal(np.where(defined, cols, 0), r["cols"])
+    assert ref.equal(np.where(defined, vals, 0), r["vals"])
     assert np.all(cols[~defined] == 77)
 
 
@@ -192,7 +181,7 @@ def test_convert_to_hybrid_matches_reference(orc, kind, strategy):
     orc("csr_convert_to_hybrid_%s_i32" % vt, n, rp, ci, va, ell_lim, n, ec, ev, crp, cr, cc, cv)
     for a, b in ((ec, r["cols"]), (ev, r["vals"]), (cr, r["coo_rows"]), (cc, r["coo_cols"]),
                  (cv, r["coo_vals"])):
-        assert np.array_equal(a, b)
+        assert ref.equal(a, b)
 
 
 @pytest.mark.parametrize("vt", ["f64", "f32"])
@@ -206,7 +195,7 @@ def test_sort_by_column_index_matches_reference(orc, vt):
         ci2[s:e], va2[s:e] = ci[s:e][perm], va[s:e][perm]
     r = ref.convert("sort", rp, ci2, va2, m)
     orc("csr_sort_by_column_index_%s_i32" % vt, n, rp, ci2, va2)
-    assert np.array_equal(ci2, r["cols"]) and np.array_equal(va2, r["vals"])
+    assert ref.equal(ci2, r["cols"]) and ref.equal(va2, r["vals"])
     assert np.array_equal(ci2, ci) and np.array_equal(va2, va)
 
 
@@ -312,4 +301,4 @@ def test_ir_and_chebyshev_loops_bit_identical_to_reference(kind, extra, precond,
         xo, ito, stop = orc_solve(kind, vt, rp, ci, va, b, x0, precond, jac, max_iters=60,
                                   reduction=red, iter_first=iter_first, **extra)
         assert itr == ito
-        assert np.array_equal(xr, xo, equal_nan=True)  # a diverging run must diverge alike
+        assert ref.equal(xo, xr, equal_nan=True)  # a diverging run must diverge alike

@@ -53,20 +53,9 @@ def true_rel_res(rp, ci, va, b, x):
 
 
 def ref_jacobi(vt, rp, ci, va, max_bs, bp):
-    """inverted blocks for the oracle: from the real reference when oracle/_ref exists,
-    else the scalar inverse computed here (block case then skipped)"""
-    from oracle import ref
-    if ref.available():
-        return ref.jacobi_generate(rp, ci, va, max_bs, bp)
-    if max_bs == 1:
-        n = len(rp) - 1
-        d = np.ones(n, VT[vt])
-        for r in range(n):
-            for k in range(rp[r], rp[r + 1]):
-                if ci[k] == r:
-                    d[r] = va[k]
-        return dict(blocks=(1 / d).astype(VT[vt]))
-    pytest.skip("block-Jacobi oracle needs oracle/_ref")
+    """inverted blocks for the oracle: the real reference's (tests/reference.py)"""
+    from tests import reference
+    return reference.jacobi_generate(rp, ci, va, max_bs, bp)
 
 
 @pytest.mark.parametrize("kind", ["cg", "bicgstab", "gmres", "fcg", "cgs"])
@@ -113,9 +102,7 @@ def test_solver_matches_oracle(hexec, kind, precond, vt, fused):
 def test_block_jacobi_with_detected_blocks(hexec):
     """Jacobi::build().with_max_block_size(4) WITHOUT block pointers: find_blocks on the device
     must reproduce the reference's blocks, so CG + block Jacobi takes the oracle's path."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("needs oracle/_ref")
+    from tests import reference as ref
     vt = "f64"
     # 2x2 block structure: a 2-D Laplacian expanded by kron(A, [[2,1],[1,2]]) has row pairs
     # with identical patterns

@@ -1,7 +1,7 @@
 """BiCG and its transposes (SURVEY.md 8f rank 3) without a GPU:
   * the oracle restatement of csr::transpose, jacobi::transpose_jacobi, the bicg kernels and the
-    BiCG loop against the REAL reference (oracle/_ref: Csr::transpose, Jacobi::transpose,
-    solver::Bicg with identity / scalar / block Jacobi);
+    BiCG loop against the REAL reference (oracle/_ref, or its recorded answers: Csr::transpose,
+    Jacobi::transpose, solver::Bicg with identity / scalar / block Jacobi);
   * a copy of ginkgo_b200/csrc/bicg_transpose.cu compiled for the host against the oracle, bit
     for bit (radix passes, chunk boundaries, empty rows / columns, duplicates, strides).
 The GPU runs of the same bodies are in tests/test_zzz_dist_assembly_gpu.py."""
@@ -14,6 +14,7 @@ import pytest
 
 import workloads as W
 from tests import helpers as H
+from tests import reference
 from tests.helpers import VT
 from tests.test_kernel_sources_cpu import KernelSourceBackend
 
@@ -42,13 +43,6 @@ def ksrc(tmp_path_factory, request):
     return KernelSourceBackend(ctypes.CDLL(so))
 
 
-def ref_or_skip():
-    from oracle import ref
-    if not ref.available() or not hasattr(ref.lib(), "refshim_csr_transpose"):
-        pytest.skip("needs oracle/_ref with the transpose / BiCG shim functions")
-    return ref
-
-
 def random_csr(rng, n, m, max_row, vt="f64", it="i32", sort=False):
     """rows of random length with duplicate and (unless sort) unsorted columns, some rows empty"""
     lens = rng.integers(0, max_row + 1, n)
@@ -75,13 +69,12 @@ def transpose(be, rp, ci, va, m, vt, it):
 @pytest.mark.parametrize("vt", ["f64", "f32"])
 @pytest.mark.parametrize("n,m,max_row", [(57, 43, 9), (300, 1000, 20), (1, 5, 4), (40, 1, 3)])
 def test_oracle_transpose_is_the_reference_transpose(orc, vt, n, m, max_row):
-    ref = ref_or_skip()
     rng = np.random.default_rng(n * 7 + m)
     rp, ci, va = random_csr(rng, n, m, max_row, vt)
-    want = ref.csr_transpose(rp, ci, va, m)
+    want = reference.csr_transpose(rp, ci, va, m)
     got = transpose(orc, rp, ci, va, m, vt, "i32")
     for a, b in zip(got, want):
-        assert np.array_equal(a, b)
+        assert reference.equal(a, b)
 
 
 @pytest.mark.parametrize("vt", ["f64", "f32"])
@@ -128,7 +121,7 @@ def _block_entries(j):
 @pytest.mark.parametrize("vt", ["f64", "f32"])
 @pytest.mark.parametrize("max_bs", [3, 8, 32])
 def test_jacobi_transpose_is_the_reference_transpose(orc, ksrc, vt, max_bs):
-    ref = ref_or_skip()
+    ref = reference
     rp, ci, va = W.laplace(9, 2, vdtype=VT[vt])
     va = va.copy()
     rng = np.random.default_rng(max_bs)
@@ -147,7 +140,7 @@ def test_jacobi_transpose_is_the_reference_transpose(orc, ksrc, vt, max_bs):
 @pytest.mark.parametrize("vt", ["f64", "f32"])
 @pytest.mark.parametrize("precond", [0, 1, 2])
 def test_oracle_bicg_is_the_reference_bicg(vt, precond):
-    ref = ref_or_skip()
+    ref = reference
     rp, ci, va = W.laplace(12, 2, vdtype=VT[vt])
     rng = np.random.default_rng(5)
     va = va.copy()
@@ -165,7 +158,7 @@ def test_oracle_bicg_is_the_reference_bicg(vt, precond):
         xo, ito, _ = H.orc_solve("bicg", vt, rp, ci, va, b, x0, precond, jac, max_iters=150, reduction=red,
                                  iter_first=iter_first)
         assert ito == itr and ito > 5
-        assert np.array_equal(xo, xr)
+        assert reference.equal(xo, xr)
 
 
 @pytest.mark.parametrize("vt", ["f64", "f32"])
